@@ -203,6 +203,22 @@ def exact_solve(cfg, limit_s):
             "wall_s": round(time.perf_counter() - t0, 2), "time_limit_s": limit_s}
 
 
+def dump_outputs(out_dir, sess, keys, reps, viol, obj, moves):
+    """Writes what the last timed step handed its caller as float64 .npy files, so that two builds can be compared
+    output for output: the base assignment it left (`replicas`, [P, RF], leader first), that base's
+    (violation, objective, moves) (`base_totals`) and, where the path returns them, each round's winning key
+    (`round_winners`, [rounds, 3]).  The keys are packed 64-bit words, so they are stored unpacked into
+    (violation, objective, candidate index), which float64 holds exactly."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"replicas": reps, "base_totals": [viol, obj, moves]}
+    if keys is not None:
+        arrays["round_winners"] = [sess.unpack_key(k) for k in keys]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -251,8 +267,14 @@ def main():
                     help="full evaluator of the search kernel: auto = the engine's default (column-major where the layout allows)")
     ap.add_argument("--collective", default="p2p", choices=["p2p", "nccl"],
                     help="N>1: per-round min inside the kernel over NVLink peer memory (p2p) or NCCL all-reduce")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float64; inputs are seeded)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the GPU path; the reference arm has none to write")
         return reference_arm(args)
 
     # stdout carries exactly ONE JSON line: whatever libraries print there while the bench runs (NCCL's version
@@ -373,7 +395,7 @@ def main():
     for k in range(args.steps):
         flush.fill_(k & 0xFF)                                # L2 flush between timed steps (outside the events)
         ev[k][0].record()
-        step(args.warmup + k)
+        last = step(args.warmup + k)
         ev[k][1].record()
     barrier()
     sampler.mark_end()
@@ -387,6 +409,8 @@ def main():
     n_total = args.steps * ROUNDS * gsize
     value = n_total / (ms * 1e-3)
     reps, viol, obj, moves = sess.get_base()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sess, None if last is None else last[0], reps, viol, obj, moves)
 
     # N > 1, untimed: the exchange cost at the small rounds a search for quality uses (32,768 candidates per
     # GPU and round), device-timed, max over ranks
