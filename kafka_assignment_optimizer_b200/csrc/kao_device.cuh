@@ -10,9 +10,6 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <type_traits>
-#ifndef KAO_LOCKSTEP
-#define KAO_LOCKSTEP 1
-#endif
 
 #include <stdint.h>
 

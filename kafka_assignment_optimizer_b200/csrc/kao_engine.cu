@@ -24,7 +24,7 @@
 #define KAO_DECL_FULL(W, NPH, R, O)                                             \
     extern template __global__ void KAO_ROUND_KERNEL(W, NPH, R, O);            \
     extern template __global__ void KAO_PERSISTENT_KERNEL(W, NPH, R, O, threads_for<W>(), false);
-#define KAO_DECL_DELTA(W, NPH, R, O) extern template __global__ void KAO_PERSISTENT_KERNEL(W, NPH, R, O, KAO_THREADS_DELTA, true);
+#define KAO_DECL_DELTA(W, NPH, R, O) extern template __global__ void KAO_PERSISTENT_KERNEL(W, NPH, R, O, kThreadsDelta, true);
 KAO_FOR_CFGS_NARROW(KAO_DECL_FULL, 1, 5) KAO_FOR_CFGS_NARROW(KAO_DECL_FULL, 2, 5)
 KAO_FOR_CFGS_WIDE(KAO_DECL_FULL, 4, 5) KAO_FOR_CFGS_WIDE(KAO_DECL_FULL, 8, 5)
 KAO_FOR_CFGS_NARROW(KAO_DECL_DELTA, 1, 5) KAO_FOR_CFGS_NARROW(KAO_DECL_DELTA, 2, 5)
@@ -187,11 +187,9 @@ struct kao_handle {
     Params prm{};
     SmemPlan plan{};
     int threads = 0, grid = 0;
-    // column-major full evaluator (kao_set_evaluator): layout supported, selected (the default wherever it
-    // applies), its shared-memory plan
+    // column-major full evaluator (kao_set_evaluator): layout supported, selected (the default wherever it applies)
     bool trans_ok = false;
     int evaluator = KAO_EVAL_ROW_MAJOR;
-    SmemPlan plan_t{};
     // schedule of the column-major evaluator (kao_set_schedule): barrier form, popcount compression per
     // stream, threads per CTA.  Same results whatever the schedule.
     int sch_sync = KAO_SCHEDULE_DEFAULT_SYNC, sch_pop = KAO_SCHEDULE_DEFAULT_POP, sch_threads = KAO_SCHEDULE_DEFAULT_THREADS;
@@ -265,7 +263,7 @@ template <bool kDelta> struct LaunchPersistent {
     template <class Cfg> cudaError_t run(kao_handle *h, const PersistArgs &a) const
     {
         {
-            constexpr int T = kDelta ? KAO_THREADS_DELTA : cfg_threads<Cfg>();
+            constexpr int T = kDelta ? kThreadsDelta : cfg_threads<Cfg>();
             auto kern = search_persistent_kernel<Cfg, T, kDelta>;
             static bool done[64] = {};
             cudaError_t e = set_smem_attr<Cfg>(h, reinterpret_cast<const void *>(kern), done);
@@ -403,7 +401,7 @@ static int create_impl(const kao_problem *pb, int32_t device, kao_handle *h)
     }
     const HostModel &m = h->hm;
     const int W = m.W, Ppad = m.Ppad;
-    h->threads = W <= 2 ? KAO_THREADS : KAO_THREADS_WIDE;
+    h->threads = W <= 2 ? kThreads : kThreadsWide;
     h->plan = make_plan(W, Ppad, h->threads / 32, m.nplanes > 0 ? m.nplanes * W : 4, m.P, m.RF, m.nplanes > 0);
     if (h->plan.total > 227u * 1024u && m.nplanes > 0) {
         // mask planes + one-hot plane do not fit next to the base: score with packed entries / the dense table
@@ -415,9 +413,8 @@ static int create_impl(const kao_problem *pb, int32_t device, kao_handle *h)
     // column-major evaluator: 8-slot rack fields, C7 = "at most one replica per rack", an objective that fits
     // eight term planes (kao_host.hpp); its two transposed planes (2 * W words per partition) and the term planes
     // take the place of the objective table.  It is the default full evaluator wherever it applies.
-    h->plan_t = make_plan_t(W, Ppad, KAO_THREADS, m.P, m.RF);
     h->trans_ok = W <= 2 && m.hi1 && m.log2S == 3 && m.z_ok &&
-                  column_major_fits(W, Ppad, 1024, m.P, m.RF);     // incl. the inverted lists of its per-thread generator
+                  column_major_fits(W, Ppad, 1024, m.P, m.RF);     // sized for the largest schedule (1024 threads)
     if (h->trans_ok) h->evaluator = KAO_EVAL_COLUMN_MAJOR;
     if (const char *env = std::getenv("KAO_EVALUATOR"))       // "row" forces the row-major evaluator (measurements)
         if (std::strcmp(env, "row") == 0) h->evaluator = KAO_EVAL_ROW_MAJOR;
@@ -544,7 +541,7 @@ static bool check_round_args(uint32_t round_size) { return round_size >= 2 && ro
 static bool delta_fits(const kao_handle *h)
 {
     if (h->hm.W <= 2) return true;                              // the session's own plan (validated at kao_create)
-    return make_plan_delta_wide(h->hm.W, h->hm.Ppad, KAO_THREADS_DELTA, h->hm.P, h->hm.RF).total <= 227u * 1024u;
+    return make_plan_delta_wide(h->hm.W, h->hm.Ppad, kThreadsDelta, h->hm.P, h->hm.RF).total <= 227u * 1024u;
 }
 
 static int reserve_keys(kao_handle *h, uint32_t rounds)

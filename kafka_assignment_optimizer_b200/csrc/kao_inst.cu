@@ -11,7 +11,7 @@
 #define KAO_INST_FULL(W, NPH, R, O)                                      \
     template __global__ void KAO_ROUND_KERNEL(W, NPH, R, O);            \
     template __global__ void KAO_PERSISTENT_KERNEL(W, NPH, R, O, threads_for<W>(), false);
-#define KAO_INST_DELTA_K(W, NPH, R, O) template __global__ void KAO_PERSISTENT_KERNEL(W, NPH, R, O, KAO_THREADS_DELTA, true);
+#define KAO_INST_DELTA_K(W, NPH, R, O) template __global__ void KAO_PERSISTENT_KERNEL(W, NPH, R, O, kThreadsDelta, true);
 
 #if KAO_INST_MODE == 2
 #if KAO_INST_W > 2

@@ -13,14 +13,11 @@
 
 using namespace kao;
 
-#ifndef KAO_THREADS
-#define KAO_THREADS 768
-#endif
-#ifndef KAO_THREADS_WIDE
-#define KAO_THREADS_WIDE 256
-#endif
-#define KAO_THREADS_DELTA 512
-template <int W> constexpr int threads_for() { return W <= 2 ? KAO_THREADS : KAO_THREADS_WIDE; }
+// threads per CTA: row-major full evaluation (rows of up to 64 slots / wider rows), delta evaluation
+constexpr int kThreads = 768;
+constexpr int kThreadsWide = 256;
+constexpr int kThreadsDelta = 512;
+template <int W> constexpr int threads_for() { return W <= 2 ? kThreads : kThreadsWide; }
 // threads per CTA of the full-evaluation kernels of a configuration (column-major schedules may choose)
 template <class Cfg> constexpr int cfg_threads()
 {
@@ -148,11 +145,7 @@ search_round_kernel(Params d, SmemPlan plan, uint64_t seed, uint32_t round, uint
 #pragma unroll
         for (int i = 0; i < kMaxOps; ++i) { ps.p[i] = -1; ps.ld[i] = 0xFF; }
         if (live) gen.run(seed, round, idx, round_size, ps, no_rows);
-#if KAO_LOCKSTEP
         __syncthreads();
-#else
-        __syncwarp();
-#endif
         if (live) {
             int viol, obj;
             eval_candidate<Cfg, true>(d, s_bits, s_leader, s_sw, s_cs, ps, gen.prow, lane, viol, obj);
@@ -497,7 +490,7 @@ search_persistent_kernel(Params d, SmemPlan plan, uint64_t seed, uint32_t first_
             if (all_keys) return;                                   // key dump only: the base stays as it is
         } else if constexpr (Cfg::kTrans) {
             // ---- column-major evaluator: candidates are generated 32 at a time, one per LANE (per-thread
-            // generator over the round's inverted lists), then evaluated in full one after the other by the warp
+            // generator scanning the transposed planes), then evaluated in full one after the other by the warp
             Gen<W, true, true> tg;        // compact code (row_kth keeps its loop), same candidates
             tg.bitsT = s_bits; tg.leader = s_leader; tg.cs = s_cs; tg.d = &d; tg.prow = nullptr; tg.lane = 0;
             tg.D = s_D; tg.DL = s_DL; tg.nD = s_counts[0]; tg.nL = s_counts[1];
@@ -641,7 +634,6 @@ search_persistent_kernel(Params d, SmemPlan plan, uint64_t seed, uint32_t first_
         // the winner becomes the base: every CTA patches its own shared-memory copy
         if (warp == 0) {
             const unsigned long long k = __ldcg(keys + t);
-#if !defined(KAO_NO_PATIENCE)
             if (lane == 0) {
                 // early stop (same decision in every CTA and on every rank: it only depends on the keys)
                 const unsigned long long vc = k >> kIdxBits;
@@ -650,7 +642,6 @@ search_persistent_kernel(Params d, SmemPlan plan, uint64_t seed, uint32_t first_
                 if (blockIdx.x == 0 && pp.rounds_run) *pp.rounds_run = t + 1;
                 if (blockIdx.x == 0 && pp.carry) { pp.carry[0] = s_red[kWarps + 1]; pp.carry[1] = s_red[kWarps + 2]; }
             }
-#endif
             if (kDelta && lane == 0) {
                 int *s_base = reinterpret_cast<int *>(smem + plan.off_totals) + 544;
                 const uint32_t kv = key_violation(k, d.key_obj_bits);
@@ -719,9 +710,7 @@ search_persistent_kernel(Params d, SmemPlan plan, uint64_t seed, uint32_t first_
         }
         __syncthreads();
         rebuild_lists<THREADS>(s_bits, s_leader, d.homeT, d.P, d.Ppad, s_D, s_DL, s_counts, s_scan);
-#if !defined(KAO_NO_PATIENCE)
         if (s_red[kWarps]) break;
-#endif
     }
 }
 
